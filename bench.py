@@ -6,14 +6,17 @@ T_text=150) synthetic text, exactly 800 decoder frames per row (gate_threshold =
 gate never fires, max_decoder_steps = 800; SURVEY.md section 8(d)) -> encoder, 800-step persistent
 decoder, postnet.  51,200 mel frames per GPU per step.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
   value : frames/s with the text ids already resident in HBM (device tensors through the nn.Module API)
   e2e   : frames/s through the C-ABI t2_infer_host with HOST buffers (pinned text in, mel_postnet out)
   roofline     : the persistent decoder kernel, algorithmic FLOPs (38,350,592 per frame) / CUDA-event time
   cpu_baseline : the oracle port (oracle/tacotron2_oracle.py, torch CPU, all host threads) on a bounded sample
-  --impl reference : the same metric from the CPU oracle port alone (the reference is pure Python and
-                     /root/reference does not exist on the GPU box; DESIGN.md "reference arm")
+  --impl reference : the same metric from the CPU oracle port alone (the reference is pure Python; DESIGN.md
+                     "reference arm")
+  --dump-outputs DIR : after the timed steps, what the last timed Tacotron2.inference returned (rank 0's batch) as
+                       DIR/<name>.npy, 63.7 MB in all; text, weights and dropout seeds are fixed, so two builds run with
+                       the same arguments can be compared output for output
 """
 import argparse
 import json
@@ -385,6 +388,15 @@ def eager_gpu_context():
         return {"unavailable": str(e)[:120]}
 
 
+def dump_outputs(out_dir, arrays):
+    """Writes name -> tensor as out_dir/<name>.npy: floating-point tensors as float32, integer ones as float64."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (t.float() if t.is_floating_point() else t.double()).numpy())
+
+
 def _launch_counter():
     from tacotron2_b200 import _capi
     return _capi.lib().t2_kernel_launch_count
@@ -399,14 +411,20 @@ def main():
     ap.add_argument("--decoder-impl", default="auto", choices=["auto", "stepwise", "persistent"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the train / config5 / eager_gpu blocks (A/B runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm has none")
         run_reference(args, rank)
         return
     args.warmup = max(args.warmup, 3)
+    # the engine's Philox dropout seeds derive from torch.initial_seed(), which is random per process unless set: fixed,
+    # runs with the same arguments compute the same outputs
+    torch.manual_seed(1234)
 
     import torch.distributed as dist
     import tacotron2_b200 as t2
@@ -453,12 +471,14 @@ def main():
 
     import contextlib
 
+    last_out = None
+
     def step_device():
+        nonlocal last_out
         # the reference prints "Warning! Reached max decoder steps" to stdout (model.py:446); this
         # workload reaches the cap by construction, keep stdout for the single JSON line
         with torch.no_grad(), contextlib.redirect_stdout(sys.stderr):
-            out = model.inference(text_dev)
-        return out
+            last_out = model.inference(text_dev)
 
     out_host = None
 
@@ -480,6 +500,10 @@ def main():
     launches0 = L.t2_kernel_launch_count()
     ms_dev = timed(step_device, args.steps)
     launches = L.t2_kernel_launch_count() - launches0
+    if args.dump_outputs and rank == 0:      # before any other call can reuse the engine's buffers
+        dump_outputs(args.dump_outputs, dict(zip(("mel_outputs", "mel_outputs_postnet", "gate_outputs", "alignments"), last_out),
+                                             mel_lengths=model.mel_lengths))
+    last_out = None
     barrier()
     ms_e2e = timed(step_host, args.steps)
     barrier()

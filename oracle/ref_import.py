@@ -1,10 +1,9 @@
 """TEST INFRASTRUCTURE ONLY -- never imported by the product path.
 
-Imports the *unmodified* reference ``/root/reference/model.py`` in the build
-container so that (a) the CPU restatement in ``oracle/tacotron2_oracle.py`` can be
-pinned against it and (b) golden vectors can be generated for ``tests/golden``.
-``/root/reference`` does not exist on the GPU box, so nothing that runs there may
-import this module (tests that use it skip when the directory is absent).
+Imports the *unmodified* reference ``model.py`` from a checkout of NVIDIA/tacotron2
+named by ``T2_REFERENCE_DIR`` so that golden vectors can be generated for
+``tests/golden`` (``tools/make_golden.py``); those fixtures are what pin the CPU
+restatement in ``oracle/tacotron2_oracle.py`` and the CUDA path.  No test imports it.
 
 Four non-invasive shims (SURVEY.md section 8(c)):
   1. stub ``librosa`` (layers.py:2, stft.py:38, audio_processing.py:4 import it; it is
@@ -20,11 +19,11 @@ import sys
 import types
 from types import SimpleNamespace
 
-REFERENCE_DIR = os.environ.get("T2_REFERENCE_DIR", "/root/reference")
+REFERENCE_DIR = os.environ.get("T2_REFERENCE_DIR", "")
 
 
 def reference_available():
-    return os.path.isfile(os.path.join(REFERENCE_DIR, "model.py"))
+    return bool(REFERENCE_DIR) and os.path.isfile(os.path.join(REFERENCE_DIR, "model.py"))
 
 
 def default_hparams(**overrides):
@@ -59,7 +58,7 @@ def import_reference_model():
     if _ref_model is not None:
         return _ref_model
     if not reference_available():
-        raise RuntimeError("reference tree not present at %s" % REFERENCE_DIR)
+        raise RuntimeError("no reference checkout at T2_REFERENCE_DIR=%r" % REFERENCE_DIR)
     for name in ("librosa", "librosa.filters", "librosa.util"):
         if name not in sys.modules:
             m = types.ModuleType(name)

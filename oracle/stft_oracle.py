@@ -8,9 +8,9 @@ CPU restatement of the log-mel extraction TacotronSTFT.mel_spectrogram (SURVEY.m
     stft.py:69-94     transform: reflect-pad by n/2 on both sides, conv1d with stride = hop, magnitude
     audio_processing.py:78-84  dynamic_range_compression
 
-Pinning: the STFT part is checked against the reference's own ``stft.STFT`` executed in the build container
-(tests/test_oracle_vs_reference.py, with functional stand-ins for the two librosa.util helpers stft.py imports) and against
-the committed fixture tests/golden/stft_mag.npz produced by it.  The mel filterbank is ``librosa.filters.mel`` of
+Pinning: the STFT part is checked against the committed fixtures tests/golden/stft_mag.npz and stft_mag_settings.npz
+produced by the reference's own ``stft.STFT`` (tools/make_golden.py, with functional stand-ins for the two librosa.util
+helpers stft.py imports).  The mel filterbank is ``librosa.filters.mel`` of
 librosa 0.6.0 (requirements.txt:5) -- a third-party dependency that is NOT in this image: ``mel_filterbank`` restates its
 published algorithm (Slaney mel scale, htk=False; area normalisation norm=1) and is **parity unpinned** against librosa
 itself; it is anchored only by its defining properties (tests/test_oracle_golden.py).

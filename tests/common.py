@@ -116,3 +116,37 @@ def rel_err(a, b):
     a = a.detach().double().cpu(); b = b.detach().double().cpu()
     den = float(b.abs().max())
     return float((a - b).abs().max()) / (den if den > 0 else 1.0)
+
+
+def tensor_digest(t):
+    """SHA-256 of a tensor's dtype, shape and bytes: equal digests <=> torch.equal with the same dtype.  Lets a fixture pin
+    large exact outputs (initial weights, collated batches) in a few bytes."""
+    import hashlib
+    t = t.detach().cpu().contiguous()
+    h = hashlib.sha256(("%s %s " % (t.dtype, tuple(t.shape))).encode())
+    h.update(t.numpy().tobytes())
+    return h.hexdigest()
+
+
+def stft_inputs(seed=0, n=6000):
+    """Two seeded test signals in [-1, 1]: two sines plus noise, and clipped noise."""
+    g = torch.Generator().manual_seed(seed)
+    t = torch.arange(n) / 22050.0
+    return torch.stack([0.3 * torch.sin(2 * math.pi * 220 * t) + 0.2 * torch.sin(2 * math.pi * 1870 * t) + 0.05 * torch.randn(n, generator=g),
+                        (0.5 * torch.randn(n, generator=g)).clamp(-1, 1)])
+
+
+def collate_batches(n_trials=20):
+    """Ragged (text, mel) batches for TextMelCollate: a fixed batch of five, then for n_frames_per_step = 1 and 2 in turn
+    `n_trials` random batches (ties in the text lengths included).  Returns (fixed, {1: [...], 2: [...]})."""
+    g = torch.Generator().manual_seed(0)
+    fixed = [(torch.randint(1, 148, (n_text,), generator=g), torch.randn(80, n_mel, generator=g))
+             for n_text, n_mel in [(7, 13), (12, 5), (3, 21), (12, 9), (1, 1)]]
+    trials = {}
+    for nfs in (1, 2):
+        trials[nfs] = []
+        for _ in range(n_trials):
+            n = int(torch.randint(1, 9, (1,), generator=g))
+            trials[nfs].append([(torch.randint(1, 148, (int(torch.randint(1, 12, (1,), generator=g)),), generator=g),
+                                 torch.randn(80, int(torch.randint(1, 30, (1,), generator=g)), generator=g)) for _ in range(n)])
+    return fixed, trials

@@ -1,102 +1,59 @@
-"""CPU, build container only: run the unmodified reference model.py live against the oracle on
-fresh random inputs (skipped where /root/reference is absent, e.g. on the GPU box)."""
-import pytest
+"""CPU: the oracle against outputs of the unmodified reference (model.py, loss_function.py, stft.py) stored under
+tests/golden by tools/make_golden.py refs."""
+import numpy as np
 import torch
 
 from oracle import tacotron2_oracle as O
-from oracle.ref_import import (MaskInjector, default_hparams, import_reference_model,
-                               injected_dropout, reference_available)
-from tests.common import keep_mask, rand_text, rel_err, synth_state_dict
+from tests.common import keep_mask, rand_text, rel_err, stft_inputs, synth_state_dict, weights_checksum
+from tests.test_oracle_golden import check_grads_vs_fixture, grad_inputs, load, oracle_train_step
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="reference tree not present")
+STFT_SETTINGS = ((1024, 256, 1024), (800, 200, 800), (512, 128, 400))     # (filter_length, hop_length, win_length)
 
 
 def test_reference_inference_b1_live():
-    ref = import_reference_model()
+    """The reference's own Tacotron2.inference at B=1 (its stop loop, 12 steps, injected prenet masks)."""
+    g = load("ref_inference_b1_t19")
     sd = synth_state_dict(5, gate_bias=-10.0, scale=2.0)
-    model = ref.Tacotron2(default_hparams()); model.load_state_dict(sd); model.eval()
-    model.decoder.max_decoder_steps = 12
+    assert abs(weights_checksum(sd) - float(g["wsum"])) < 1e-6 * float(g["wsum"]), "weight generator drifted"
     text = rand_text(1, 19, 3); keep = keep_mask((12, 2, 1, 256), 0.5, 4)
-    masks = [keep[t, l].bool() for t in range(12) for l in range(2)]
-    with torch.no_grad(), injected_dropout(ref, MaskInjector(masks)):
-        r = model.inference(text)
     with torch.no_grad():
         mel, post, gate, align, lengths = O.tacotron2_inference(sd, text, keep, 0.5, 12)
-    assert int(lengths[0]) == r[0].shape[2] == 12
-    for a, b in zip((mel, post, gate, align), r):
-        assert rel_err(a, b) < 2e-5
+    assert int(lengths[0]) == g["mel"].shape[2] == 12
+    for a, k in zip((mel, post, gate, align), ("mel", "mel_post", "gate", "align")):
+        assert rel_err(a, torch.from_numpy(g[k])) < 2e-5, k
 
 
 def test_reference_state_dict_layout():
     """The 84 keys / shapes the boundary must reproduce (SURVEY.md section 8(b1))."""
     from tests.common import state_dict_shapes
-    ref = import_reference_model()
-    sd = ref.Tacotron2(default_hparams()).state_dict()
+    g = load("ref_init_seed1234")
     want = state_dict_shapes()
-    assert list(sd.keys()) == list(want.keys())
-    for k, v in sd.items():
-        assert tuple(v.shape) == tuple(want[k]), k
+    assert g["keys"].tolist() == list(want.keys())
+    for k, s in zip(g["keys"].tolist(), g["shapes"].tolist()):
+        assert tuple(int(n) for n in s.split(",") if n) == tuple(want[k]), k
 
 
 def test_reference_training_step_gradients_live():
     """Full training step (forward + Tacotron2Loss + backward) of the unmodified reference vs torch autograd through
-    the oracle: every parameter gradient, full tensors (the committed fixtures tests/golden/grad_*.npz keep samples)."""
-    import importlib.util
-    from tests.test_oracle_golden import oracle_train_step
-    ref = import_reference_model()
-    spec = importlib.util.spec_from_file_location("ref_loss_function", "/root/reference/loss_function.py")
-    lf = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(lf)
-    B, T, Tm, seed = 3, 15, 8, 91
-    sd = synth_state_dict(4321, scale=2.0)
-    g = torch.Generator().manual_seed(seed)
-    text = rand_text(B, T, seed + 1)
-    tl = torch.sort(torch.randint(T // 3, T + 1, (B,), generator=g), descending=True)[0]
-    tl[0] = T
-    ol = torch.randint(Tm // 3, Tm + 1, (B,), generator=g)
-    ol[1] = Tm
-    mels = torch.randn(B, 80, Tm, generator=g)
-    gt = torch.zeros(B, Tm)
-    for i, n in enumerate(ol.tolist()):
-        mels[i, :, n:] = 0.0
-        gt[i, n - 1:] = 1.0
-    m = dict(pk=keep_mask((Tm + 1, 2, B, 256), 0.5, seed + 2), ak=keep_mask((Tm, B, 1024), 0.1, seed + 3),
-             dk=keep_mask((Tm, B, 1024), 0.1, seed + 4), ek=keep_mask((3, B, 512, T), 0.5, seed + 5),
-             qk4=keep_mask((4, B, 512, Tm), 0.5, seed + 6), qk1=keep_mask((B, 80, Tm), 0.5, seed + 7))
-    model = ref.Tacotron2(default_hparams())
-    model.load_state_dict(sd)
-    model.train()
-    masks = [m["ek"][i].bool() for i in range(3)] + [m["pk"][:, 0].bool(), m["pk"][:, 1].bool()]
-    for t in range(Tm):
-        masks += [m["ak"][t].bool(), m["dk"][t].bool()]
-    masks += [m["qk4"][i].bool() for i in range(4)] + [m["qk1"].bool()]
-    with injected_dropout(ref, MaskInjector(masks)):
-        out = model((text, tl, mels, int(tl.max()), ol))
-    loss = lf.Tacotron2Loss()(out, (mels, gt))
-    loss.backward()
+    the oracle: the loss, and per parameter the gradient's sum / abs-sum / max and 512 sampled entries."""
+    g = load("grad_train_b3_t15_m8")
+    sd, text, tl, ol, mels, gt, m = grad_inputs(g)
     o_loss, _, o_grads = oracle_train_step(sd, text, tl, ol, mels, gt, m, True)
-    assert abs(float(loss) - float(o_loss)) < 1e-5 * abs(float(loss))
-    for k, p in model.named_parameters():
-        if float(p.grad.abs().max()) < 1e-5:      # conv biases in front of a training-mode BatchNorm: rounding noise
-            assert float(o_grads[k].abs().max()) < 1e-4
-            continue
-        assert rel_err(o_grads[k], p.grad) < 1e-4, k
+    assert abs(float(g["loss"]) - float(o_loss)) < 1e-5 * abs(float(g["loss"]))
+    assert set(o_grads) == {k[2:] for k in g if k.startswith("g/")}
+    check_grads_vs_fixture(o_grads, g, 1e-4)
 
 
 def test_stft_oracle_vs_reference_stft_live():
-    """oracle/stft_oracle.py against the reference's own stft.STFT executed here (functional stand-ins for the two
-    librosa.util helpers stft.py imports): the windowed Fourier basis and the magnitudes for two filter / hop settings."""
-    import os
-    import sys
-    if not os.path.isfile("/root/reference/stft.py"):
-        pytest.skip("reference tree not present")
-    sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tools"))
+    """oracle/stft_oracle.py against the reference's own stft.STFT (functional stand-ins for the two librosa.util helpers
+    stft.py imports): the windowed Fourier basis and the magnitudes for three filter / hop settings."""
     from oracle import stft_oracle as S
-    from tools.make_golden import import_reference_stft, stft_inputs
-    mod = import_reference_stft()
-    for fl, hop, win in ((1024, 256, 1024), (800, 200, 800), (512, 128, 400)):
-        ref_stft = mod.STFT(fl, hop, win)
-        assert float((ref_stft.forward_basis[:, 0, :] - torch.from_numpy(S.stft_forward_basis(fl, win))).abs().max()) < 1e-6
+    g = load("stft_mag_settings")
+    for fl, hop, win in STFT_SETTINGS:
+        basis = torch.from_numpy(S.stft_forward_basis(fl, win)).reshape(-1)
+        idx = torch.from_numpy(g["basis_index_%d" % fl]).long()
+        assert float((basis[idx] - torch.from_numpy(g["basis_%d" % fl])).abs().max()) < 1e-6
+        abs_sum = float(g["basis_abs_sum_%d" % fl])
+        assert abs(float(np.abs(S.stft_forward_basis(fl, win)).sum(dtype=np.float64)) - abs_sum) < 1e-6 * abs_sum
         y = stft_inputs(seed=fl, n=5000)
-        mag, _ = ref_stft.transform(y)
-        assert rel_err(S.stft_magnitude(y, fl, hop, win), mag) < 1e-6
+        assert rel_err(S.stft_magnitude(y, fl, hop, win), torch.from_numpy(g["mag_%d" % fl])) < 1e-6

@@ -1,5 +1,5 @@
-"""Generates tests/golden/*.npz by executing the UNMODIFIED reference model.py (build container
-only -- needs /root/reference).  Run:  python tools/make_golden.py
+"""Generates tests/golden/*.npz by executing the UNMODIFIED reference model.py (a checkout of NVIDIA/tacotron2 named by
+T2_REFERENCE_DIR).  Run:  T2_REFERENCE_DIR=<checkout> python tools/make_golden.py [stft | full | grads | refs]
 
 Every file holds the inputs' seeds, the reference outputs and a checksum of the synthetic weights
 (tests/common.synth_state_dict) so a drift of the generator is detected instead of silently
@@ -14,9 +14,10 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-from oracle.ref_import import (MaskInjector, default_hparams, import_reference_model,  # noqa: E402
+from oracle.ref_import import (REFERENCE_DIR, MaskInjector, default_hparams, import_reference_model,  # noqa: E402
                                injected_dropout)
-from tests.common import GOLDEN_DIR, keep_mask, rand_text, synth_state_dict, weights_checksum  # noqa: E402
+from tests.common import (GOLDEN_DIR, collate_batches, keep_mask, rand_text, stft_inputs, synth_state_dict,  # noqa: E402
+                          tensor_digest, weights_checksum)
 
 torch.set_num_threads(8)
 ref = import_reference_model()
@@ -167,17 +168,18 @@ def pick_gate(gate, S):
     return best
 
 
-FULL_STRIDE, FULL_TAIL, FULL_ALIGN_STRIDE = 25, 8, 100
+# frames / alignment rows kept by the full-size fixtures: sparse enough that each file stays under 1 MB
+FULL_STRIDE, FULL_TAIL, FULL_ALIGN_STRIDE = 50, 8, 200
 
 
-def full_frame_index(S):
-    return sorted(set(range(0, S, FULL_STRIDE)) | set(range(S - FULL_TAIL, S)))
+def full_frame_index(S, stride=FULL_STRIDE):
+    return sorted(set(range(0, S, stride)) | set(range(S - FULL_TAIL, S)))
 
 
 def full_infer_case(name, B, T_text, S, wseed, tseed, mseed, wscale):
     """The configuration a number is QUOTED on (BASELINE.json configs[1] / configs[4] per GPU), all S steps through the
-    reference's own modules.  Stored: every 25th frame + the last 8 of mel / mel_postnet, all gates, all mel_lengths,
-    the alignment argmax of every step and the alignment rows of every 100th step."""
+    reference's own modules.  Stored: every 50th frame + the last 8 of mel / mel_postnet, all gates, all mel_lengths,
+    the alignment argmax of every step and the alignment rows of every 200th step."""
     sd0 = synth_state_dict(wseed, gate_bias=0.0, scale=wscale)
     text = rand_text(B, T_text, tseed)
     keep = keep_mask((S, 2, B, 256), 0.5, mseed)
@@ -201,7 +203,7 @@ def full_infer_case(name, B, T_text, S, wseed, tseed, mseed, wscale):
           "gate pre-activation margin %.3e" % margin)
     save(name, B=B, T_text=T_text, max_steps=S, wseed=wseed, wscale=wscale, tseed=tseed, mseed=mseed, gate_bias=bias,
          gate_sign=sign, wsum=weights_checksum(sd), frame_index=idx, align_index=aidx, mel_masked=mel_masked[:, :, idx],
-         mel_raw=mel[:, :, idx], mel_post=post[:, :, idx], gate=gate, mel_lengths=lengths, gate_margin=margin,
+         mel_post=post[:, :, idx], gate=gate, mel_lengths=lengths, gate_margin=margin,
          align_argmax=align.argmax(-1).to(torch.int16), align_max=align.max(-1)[0], align_rows=align[:, aidx],
          memory_abs_sum=memory.double().abs().sum())
 
@@ -263,7 +265,7 @@ def grad_case(name, training, B, T_text, T_mel, wseed, seed, wscale=2.0, n_sampl
     """Full training step of the REFERENCE (forward + Tacotron2Loss + backward, autograd) with injected dropout
     masks; the fixture keeps the loss and, per parameter, sum / abs-sum / max of the gradient plus 96 sampled entries."""
     import importlib.util
-    spec = importlib.util.spec_from_file_location("ref_loss_function", "/root/reference/loss_function.py")
+    spec = importlib.util.spec_from_file_location("ref_loss_function", os.path.join(REFERENCE_DIR, "loss_function.py"))
     lf = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(lf)
     sd = synth_state_dict(wseed, scale=wscale)
@@ -299,7 +301,7 @@ def grad_case(name, training, B, T_text, T_mel, wseed, seed, wscale=2.0, n_sampl
                   wsum=weights_checksum(sd), text_lengths=tl, output_lengths=ol, mels_in=mels, gate_target=gt,
                   loss=loss.detach(), mel=out[0].detach(), mel_post=out[1].detach(), n_samples=n_samples)
     if not keep_outputs:      # full-size case: the inputs are regenerated from the seeds, outputs sub-sampled in time
-        idx = torch.tensor(full_frame_index(T_mel))
+        idx = torch.tensor(full_frame_index(T_mel, 2 * FULL_STRIDE))
         arrays.update(mel=out[0].detach()[:, :, idx], mel_post=out[1].detach()[:, :, idx], frame_index=idx, gate=out[2].detach())
         del arrays["mels_in"], arrays["gate_target"]
     for k, p_ in model.named_parameters():
@@ -349,13 +351,13 @@ def import_reference_stft():
     lu.pad_center, lu.tiny, lf.mel = pad_center, (lambda x: np.finfo(np.float32).tiny), None
     lib.util, lib.filters = lu, lf
     sys.modules.update({"librosa": lib, "librosa.util": lu, "librosa.filters": lf})
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, REFERENCE_DIR)
     try:
-        spec = importlib.util.spec_from_file_location("t2_reference_stft", "/root/reference/stft.py")
+        spec = importlib.util.spec_from_file_location("t2_reference_stft", os.path.join(REFERENCE_DIR, "stft.py"))
         mod = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(mod)
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(REFERENCE_DIR)
         for k, v in saved.items():
             sys.modules.pop(k, None)
             if v is not None:
@@ -363,11 +365,70 @@ def import_reference_stft():
     return mod
 
 
-def stft_inputs(seed=0, n=6000):
-    g = torch.Generator().manual_seed(seed)
-    t = torch.arange(n) / 22050.0
-    return torch.stack([0.3 * torch.sin(2 * np.pi * 220 * t) + 0.2 * torch.sin(2 * np.pi * 1870 * t) + 0.05 * torch.randn(n, generator=g),
-                        (0.5 * torch.randn(n, generator=g)).clamp(-1, 1)])
+STFT_SETTINGS = ((1024, 256, 1024), (800, 200, 800), (512, 128, 400))     # (filter_length, hop_length, win_length)
+
+
+def stft_settings_case():
+    """The reference's stft.STFT for three filter / hop / window settings on seeded 2-row signals: the magnitudes, and 4096
+    seeded samples plus the absolute sum of the windowed Fourier basis (the whole basis is 4 MB at filter_length 1024)."""
+    mod = import_reference_stft()
+    g = torch.Generator().manual_seed(0)
+    out = {}
+    for fl, hop, win in STFT_SETTINGS:
+        ref_stft = mod.STFT(fl, hop, win)
+        basis = ref_stft.forward_basis[:, 0, :].reshape(-1)
+        idx = torch.randint(0, basis.numel(), (4096,), generator=g)
+        mag, _ = ref_stft.transform(stft_inputs(seed=fl, n=5000))
+        out.update({"mag_%d" % fl: mag, "basis_index_%d" % fl: idx.to(torch.int32), "basis_%d" % fl: basis[idx],
+                    "basis_abs_sum_%d" % fl: basis.double().abs().sum()})
+    save("stft_mag_settings", **out)
+
+
+def import_reference_collate():
+    """The reference's data_utils.py with stand-ins for the modules it imports but TextMelCollate does not use."""
+    import importlib.util
+    import types
+    saved = {k: sys.modules.get(k) for k in ("layers", "utils", "text")}
+    try:
+        for k in saved:
+            sys.modules[k] = types.ModuleType(k)
+        sys.modules["utils"].load_wav_to_torch = sys.modules["utils"].load_filepaths_and_text = None
+        sys.modules["text"].text_to_sequence = None
+        spec = importlib.util.spec_from_file_location("t2_reference_data_utils", os.path.join(REFERENCE_DIR, "data_utils.py"))
+        mod = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(mod)
+    finally:
+        for k, v in saved.items():
+            sys.modules.pop(k, None)
+            if v is not None:
+                sys.modules[k] = v
+    return mod
+
+
+def refs_cases():
+    """Fixtures for tests/test_oracle_vs_reference.py and the reference checks of tests/test_boundary_cpu.py."""
+    # Tacotron2.inference of the reference itself at B=1, 12 steps (its own stop loop, injected prenet masks)
+    sd = synth_state_dict(5, gate_bias=-10.0, scale=2.0)
+    model = build(sd)
+    model.decoder.max_decoder_steps = 12
+    text, keep = rand_text(1, 19, 3), keep_mask((12, 2, 1, 256), 0.5, 4)
+    masks = [keep[t, l].bool() for t in range(12) for l in range(2)]
+    with torch.no_grad(), injected_dropout(ref, MaskInjector(masks)):
+        r = model.inference(text)
+    save("ref_inference_b1_t19", wsum=weights_checksum(sd), mel=r[0], mel_post=r[1], gate=r[2], align=r[3])
+    # state_dict keys / shapes, and the initial weights under torch.manual_seed(1234) as one digest per entry
+    torch.manual_seed(1234)
+    sd = ref.Tacotron2(default_hparams()).state_dict()
+    save("ref_init_seed1234", keys=np.array(list(sd)), shapes=np.array([",".join(map(str, v.shape)) for v in sd.values()]),
+         digests=np.array([tensor_digest(v) for v in sd.values()]))
+    # a whole training step (forward + Tacotron2Loss + backward) of the reference
+    grad_case("grad_train_b3_t15_m8", True, 3, 15, 8, 4321, 91, n_samples=512)
+    stft_settings_case()
+    # TextMelCollate on the batches of tests.common.collate_batches: digests of its five outputs
+    coll = import_reference_collate()
+    fixed, trials = collate_batches()
+    save("ref_collate", digests=np.array([[[tensor_digest(t) for t in coll.TextMelCollate(nfs)(b)] for b in [fixed] + trials[nfs]]
+                                          for nfs in (1, 2)]))
 
 
 def stft_case():
@@ -392,6 +453,9 @@ if __name__ == "__main__":
         if "grad64" in which:    # configs[2]: teacher-forced training step B=64, T_mel=800
             grad_case("full_grad_train_b64_t150_m800", True, 64, 150, 800, 1234, 160, wscale=1.0, n_samples=1024,
                       keep_outputs=False, ref64=True)
+        sys.exit(0)
+    if len(sys.argv) > 1 and sys.argv[1] == "refs":
+        refs_cases()
         sys.exit(0)
     if len(sys.argv) > 1 and sys.argv[1] == "grads":
         grad_case("grad_train_b4", True, 4, 24, 12, 1234, 60)
