@@ -150,6 +150,17 @@ def _check_train_rows(B, what):
                            % (what, MAX_TRAIN_ROWS, B, MAX_TRAIN_ROWS))
 
 
+MAX_TRAIN_T_ENC = 408  # longest encoder sequence the decoder backward takes: att_bwd_smem(T_enc) <= 220 KiB (decoder_backward.cu)
+
+
+def _check_train_t_enc(T_enc, what):
+    # raised before any kernel runs, so no parameter is left with a partially accumulated .grad and no BatchNorm running
+    # statistic moves for a step that cannot complete
+    if T_enc > MAX_TRAIN_T_ENC:
+        raise RuntimeError("tacotron2_b200: %s under autograd: T_enc = %d too long for the attention kernel of the decoder "
+                           "backward (at most %d encoder positions)" % (what, T_enc, MAX_TRAIN_T_ENC))
+
+
 class _EncoderFn(torch.autograd.Function):
     """Encoder.forward (model.py:173-190) [+ the embedding lookup of model.py:503 when `text` is given] as one autograd
     node: forward = fp32 conv stack + persistent BiLSTM with a stash, backward = t2_encoder_backward."""
@@ -405,6 +416,7 @@ class Decoder(_EngineOwner, nn.Module):
         params = [p_ for p_ in self.parameters()]
         if torch.is_grad_enabled() and (memory.requires_grad or any(p_.requires_grad for p_ in params)):
             _check_train_rows(memory.size(0), "Decoder.forward")
+            _check_train_t_enc(memory.size(1), "Decoder.forward")
             mel, gate, align = _DecoderFn.apply(self, memory, decoder_inputs, memory_lengths, *params)
         else:
             mel, gate, align, _ = self._teacher_forward(memory, decoder_inputs, memory_lengths, False)
@@ -528,6 +540,7 @@ class Tacotron2(_EngineOwner, nn.Module):
         grad = _wants_grad(self)
         if grad:
             _check_train_rows(text_inputs.size(0), "Tacotron2.forward")
+            _check_train_t_enc(text_inputs.size(1), "Tacotron2.forward")
         if grad:   # embedding lookup + encoder as one node (the embedding gradient comes out of t2_encoder_backward)
             named = [("embedding.weight", self.embedding.weight)] + [("encoder." + k, p_) for k, p_ in self.encoder.named_parameters()]
             memory = _EncoderFn.apply(self, [n for n, _ in named], text_inputs, None, text_lengths, self.training,
